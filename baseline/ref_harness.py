@@ -6,8 +6,7 @@ path, and nothing of this repo's engine is on the path timed here: the objects b
 `inference.StyleSinger.StyleSingerInfer` (its `StyleSinger` model + its registered `HifiGAN_NSF` vocoder), constructed
 by the reference's own constructor from checkpoint directories written in the reference's on-disk format.
 
-The reference source is found by tools/ref_import.py (/root/reference in the build container, the byte-for-byte staged
-copy under baseline/_ref/StyleSinger on the GPU box).  Inputs / checkpoints: stylesinger_b200.synth and
+The reference source is found by tools/ref_import.py (the checkout STYLESINGER_REF names).  Inputs / checkpoints: stylesinger_b200.synth and
 stylesinger_b200.hparams, which are plain Python (they do not load libstylesinger_b200.so).
 """
 import json

@@ -3,8 +3,9 @@
 
     python bench.py --gpus 1 --steps K --warmup W [--workload utt10s|batch64] [--T 100]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
-    python bench.py --impl reference ...      # CPU arm: the UNMODIFIED reference (staged under baseline/_ref by
-                                              # build(); the oracle port only if that copy is absent), host cores
+    python bench.py --impl reference ...      # CPU arm: the UNMODIFIED reference where tools/ref_import.py finds its
+                                              # sources, else the oracle port; host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
     python bench.py --workload sweep          # BASELINE.json configs[4]: T sweep, persistent vs per-launch mel sampler
 
 A "step" is one pass of the whole hot path (encoder, style adaptor + RVQ, two F0/UV diffusions, FFT
@@ -102,8 +103,8 @@ def make_workload(name, rank, world, describe_only=False):
 class CpuArm:
     """The reference's own implementation of the path on the host cores.  kind "reference": the unmodified reference
     (baseline/ref_harness.py drives its StyleSingerInfer, model and vocoder built by the reference's own loaders from
-    checkpoint directories in its on-disk format); kind "port": the oracle restatement, used only when the staged copy of
-    the reference is absent.  Neither touches libstylesinger_b200.so."""
+    checkpoint directories in its on-disk format); kind "port": the oracle restatement, used only when tools/ref_import.py
+    finds no copy of the reference.  Neither touches libstylesinger_b200.so."""
 
     def __init__(self, T, threads):
         self.T, self.threads = T, threads
@@ -117,14 +118,14 @@ class CpuArm:
                 with contextlib.redirect_stdout(sys.stderr):  # the reference prints while loading: keep stdout to the JSON line
                     self.runner = ref_harness.ReferenceRunner(T=T, device="cpu", threads=threads)
                 os.chdir(cwd)
-        except Exception as e:  # staged copy broken: say so and fall back to the port
+        except Exception as e:  # reference copy broken: say so and fall back to the port
             print(f"[bench] reference harness unavailable ({type(e).__name__}: {e}); using the oracle port", file=sys.stderr)
             self.runner = None
         self.kind = "reference" if self.runner is not None else "port"
 
     def describe(self):
         return ("unmodified reference (inference/StyleSinger.py:41-64 with explicit mel2ph; StyleSinger + HifiGAN_NSF from its "
-                "own loaders)" if self.kind == "reference" else "CPU oracle port of the reference (staged reference absent)")
+                "own loaders)" if self.kind == "reference" else "CPU oracle port of the reference (no reference copy found)")
 
     def one_pass(self, seconds, utt_idx=0):
         if self.runner is not None:
@@ -201,6 +202,32 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 60 << 20  # with the .npy headers, under 64 MB
+
+
+def dump_outputs(outdir, arrays, budget=None):
+    """Write each array as <outdir>/<name>.npy (float64 for integer arrays, float32 otherwise).  When together they exceed
+    `budget` bytes (default DUMP_BYTES), every array with more than 4096 rows keeps the same fraction of its rows, chosen by
+    np.random.default_rng(0) and sorted (so equal row counts give equal rows), and those row indices go to
+    <name>_rows.npy."""
+    budget = DUMP_BYTES if budget is None else budget
+    os.makedirs(outdir, exist_ok=True)
+    host = {}
+    for k, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        host[k] = a.astype(np.float64 if a.dtype.kind in "iub" else np.float32)
+    big = [k for k, a in host.items() if a.shape[0] > 4096]
+    small_bytes = sum(a.nbytes for k, a in host.items() if k not in big)
+    big_bytes = sum(host[k].nbytes + 8 * host[k].shape[0] for k in big)  # values + float64 row index
+    keep = min(1.0, (budget - small_bytes) / max(big_bytes, 1))
+    for k, a in host.items():
+        if k in big and keep < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * keep), replace=False))
+            np.save(os.path.join(outdir, k + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(outdir, k + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------
 def run_b200(args, rank, world, local_rank):
     import torch.distributed as dist
@@ -248,12 +275,26 @@ def run_b200(args, rank, world, local_rank):
     torch.cuda.synchronize(dev)
 
     # ---- value: device-resident inputs
+    last = {}
+
+    def value_step(s):
+        out = eng.run_device(pb_dev, seed=100 + s)
+        if s == args.steps - 1:
+            last["out"] = out
+
     clocks = ClockSampler(local_rank)
     clocks.start()
     l0 = lib.ssb_launch_count()
-    ms = timed(lambda s: eng.run_device(pb_dev, seed=100 + s), args.steps)
+    ms = timed(value_step, args.steps)
     launches = int(lib.ssb_launch_count() - l0)
     clk = clocks.stop()
+    if args.dump_outputs:
+        mel, f0, wav, fo_v = last["out"]
+        hop = eng.vocoder.hop
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     {"mel_out": mel, "f0_denorm": f0, "wav": wav.reshape(-1, hop), "wav_frame_offsets": fo_v},
+                     budget=DUMP_BYTES // world)  # every rank writes its own shard
+    del last
 
     # ---- e2e: host buffers in, host waveform out
     wav_bytes = frames * 256 * 4
@@ -284,9 +325,8 @@ def run_b200(args, rank, world, local_rank):
             return gather_waveforms_device(wav, fo_v, eng.vocoder.hop, idx, n_total, dst=0)
 
         sg_step(0)
-        sg_steps = max(1, min(args.steps, 3))
-        ms_sg = timed(sg_step, sg_steps)
-        sg = {"ms_per_step": ms_sg, "steps": sg_steps}
+        ms_sg = timed(sg_step, args.steps)
+        sg = {"ms_per_step": ms_sg, "steps": args.steps}
 
     # ---- latency regime: BASELINE.json configs[1] (one 10 s utterance) through the same public API
     lat = None
@@ -295,7 +335,7 @@ def run_b200(args, rank, world, local_rank):
         pb10 = pack_batch(u10, use_mel2ph=True, pin=True)
         for s_ in range(2):
             eng.infer_packed(pb10, seed=s_)
-        ms10 = timed(lambda s: eng.infer_packed(pb10, seed=300 + s), max(args.steps, 3))
+        ms10 = timed(lambda s: eng.infer_packed(pb10, seed=300 + s), args.steps)
         f10 = pb10.total_frames
         lat = {"workload": "utt10s: one 10 s utterance (BASELINE.json configs[1]), host buffers in/out", "frames": f10,
                "ms": ms10, "frames_per_s": f10 / (ms10 / 1000.0), "rtf": (ms10 / 1000.0) / (f10 * 256 / 48000.0)}
@@ -305,8 +345,8 @@ def run_b200(args, rank, world, local_rank):
     cond, coarse = out["diff_cond"], out["coarse_mel"]
     eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=2)
     l1 = lib.ssb_launch_count()
-    ms_mel = timed(lambda s: eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=3 + s), max(1, min(args.steps, 3)))
-    n_mel = int(lib.ssb_launch_count() - l1) // max(1, min(args.steps, 3))
+    ms_mel = timed(lambda s: eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=3 + s), args.steps)
+    n_mel = int(lib.ssb_launch_count() - l1) // args.steps
     pk = peaks()
     traffic = None  # dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernel, from the committed
     tpath = os.path.join(REPO, "profiles", "traffic.json")  # ncu --set full capture of this workload (profiles/*.md)
@@ -446,11 +486,10 @@ def run_sweep(args, rank, world, local_rank):
         for arm, grp in (("per_launch", False), ("persistent_groups", True)):
             eng.model.set_persistent_groups(grp)
             eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=2)  # warm-up
-            steps = max(1, min(args.steps, 3 if T <= 100 else 2))
             l0 = lib.ssb_launch_count()
-            ms = timed(lambda s_: eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=3 + s_), steps)
+            ms = timed(lambda s_: eng.model.mel_diffusion(cond, coarse, pb_dev.frame_offsets, seed=3 + s_), args.steps)
             tf = frames * T * MEL_STEP_FLOPS / (ms / 1000.0) / 1e12
-            row[arm] = {"ms": ms, "launches": int(lib.ssb_launch_count() - l0) // steps, "frames_per_s": frames / (ms / 1000.0),
+            row[arm] = {"ms": ms, "launches": int(lib.ssb_launch_count() - l0) // args.steps, "frames_per_s": frames / (ms / 1000.0),
                         "useful_tflops": tf, "frac_of_bf16_peak": tf / pk["bf16_tflops"],
                         "hbm_streamed_gbs": frames * T * MEL_STEP_STREAM_BYTES / (ms / 1000.0) / 1e9}
         rows.append(row)
@@ -480,7 +519,16 @@ def main():
     ap.add_argument("--sweep-T", default="25,50,100,200,500")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's mel_out, f0_denorm, wav (rows of one hop) and "
+                         "wav_frame_offsets as DIR/<name>.npy (DIR/rank<r>/ per rank when N>1; at most 64 MB over all "
+                         "ranks, a fixed seeded row sample when larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "sweep"):
+        ap.error("--dump-outputs writes the outputs of the b200 ph -> wav pass; --impl reference and --workload sweep "
+                 "do not run it")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,41 +1,19 @@
-"""stylesinger_b200/formats.py against the reference's own writers / loaders (imported by file path from /root/reference
-when it is present - it is in the build container, where the CPU suite runs - and hand-written files otherwise)."""
-import importlib.util
+"""stylesinger_b200/formats.py against the reference's own writers / loaders (their outputs on the inputs below are stored
+in tests/golden/ref_formats.npz by tools/make_golden.py formats) and against hand-written files."""
 import json
 import os
 import pickle
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
 from stylesinger_b200 import formats as F
+from tests.common import GOLDEN
 
-REF = "/root/reference"
 
-
-def _ref_module(rel, name, stubs=()):
-    path = os.path.join(REF, rel)
-    if not os.path.exists(path):
-        pytest.skip("reference sources not present")
-    added = []
-    for s in stubs:
-        if s not in sys.modules:
-            sys.modules[s] = types.ModuleType(s)
-            added.append(s)
-    prev = sys.dont_write_bytecode
-    sys.dont_write_bytecode = True  # never write into /root/reference
-    try:
-        spec = importlib.util.spec_from_file_location(name, path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-    finally:
-        sys.dont_write_bytecode = prev
-        for s in added:
-            del sys.modules[s]
-    return mod
+def _ref():
+    return np.load(os.path.join(GOLDEN, "ref_formats.npz"))
 
 
 def _tiny_sd(seed):
@@ -67,24 +45,17 @@ def test_checkpoint_selection_and_key_layouts(tmp_path):
 
 
 def test_checkpoint_loader_agrees_with_the_reference_load_ckpt(tmp_path):
-    ck = _ref_module("utils/commons/ckpt_utils.py", "ref_ckpt_utils")
-
-    class Tiny(torch.nn.Module):
-        def __init__(self):
-            super().__init__()
-            self.encoder = torch.nn.Linear(4, 3)
-            self.proj = torch.nn.Conv1d(3, 2, 3)
-
-    torch.manual_seed(0)
-    src = Tiny()
+    """Two checkpoints of a small module in one work dir: the state dict the reference's load_ckpt put into the module
+    (it picks the newest step) is what F.load_state_dict returns."""
+    g = _ref()
     d = str(tmp_path)
-    torch.save({"state_dict": {"model": src.state_dict()}, "global_step": 7}, os.path.join(d, "model_ckpt_steps_7.ckpt"))
-    torch.save({"state_dict": {"model": Tiny().state_dict()}}, os.path.join(d, "model_ckpt_steps_3.ckpt"))
-    dst = Tiny()
-    ck.load_ckpt(dst, d, "model", strict=True)  # the reference picks the newest step
+    for step in (7, 3):
+        sd = {k[len(f"ckpt{step}_"):]: torch.from_numpy(g[k]) for k in g.files if k.startswith(f"ckpt{step}_")}
+        torch.save({"state_dict": {"model": sd}, "global_step": step}, os.path.join(d, f"model_ckpt_steps_{step}.ckpt"))
+    loaded = {k[len("loaded_"):]: torch.from_numpy(g[k]) for k in g.files if k.startswith("loaded_")}
     mine, _ = F.load_state_dict(d, "model")
-    assert sorted(mine) == sorted(dst.state_dict())
-    assert all(torch.equal(mine[k], v) for k, v in dst.state_dict().items())
+    assert sorted(mine) == sorted(loaded)
+    assert all(torch.equal(mine[k], v) for k, v in loaded.items())
 
 
 def test_vocoder_checkpoint_layouts(tmp_path):
@@ -123,22 +94,21 @@ def _items(n=5):
 
 
 def test_indexed_dataset_written_by_the_reference_builder(tmp_path):
-    ids = _ref_module("utils/commons/indexed_datasets.py", "ref_indexed_datasets")
+    """<prefix>.data / .idx as the reference's IndexedDatasetBuilder wrote them for _items()."""
+    g = _ref()
     items = _items()
     prefix = str(tmp_path / "test")
-    b = ids.IndexedDatasetBuilder(prefix)
-    for it in items:
-        b.add_item(it)
-    b.finalize()
+    for ext in ("data", "idx"):
+        with open(f"{prefix}.{ext}", "wb") as f:
+            f.write(g["ids_" + ext].tobytes())
     with F.IndexedDatasetReader(prefix) as ds:
         assert len(ds) == len(items)
         for i in (3, 0, 4, 1, 2):
             got = ds[i]
             assert got["item_name"] == items[i]["item_name"] and np.array_equal(got["mel"], items[i]["mel"])
+            assert np.array_equal(got["f0"], items[i]["f0"])
         with pytest.raises(IndexError):
             ds[len(items)]
-    ref_ds = ids.IndexedDataset(prefix)
-    assert len(ref_ds) == len(items) and np.array_equal(ref_ds[2]["f0"], items[2]["f0"])
 
 
 def test_indexed_dataset_hand_written_files(tmp_path):
@@ -155,15 +125,12 @@ def test_indexed_dataset_hand_written_files(tmp_path):
 
 
 def test_norm_interp_f0_matches_the_reference():
-    pu = _ref_module("utils/pitch_utils.py", "ref_pitch_utils", stubs=("librosa",))
-    rng = np.random.default_rng(1)
-    hp = {"pitch_norm": "log", "use_uv": True}
-    for n, p0 in ((50, 0.3), (17, 0.0), (9, 1.0), (64, 0.9)):
-        f0 = rng.uniform(100, 600, n).astype(np.float32)
-        f0[rng.random(n) < p0] = 0.0
-        rf, ru = pu.norm_interp_f0(f0.copy(), hp)
+    """The reference's norm_interp_f0 (pitch_norm log, use_uv) on tracks with 0 %, some and all frames unvoiced."""
+    g = _ref()
+    for i in range(4):
+        f0 = g[f"f0_{i}"]
         mf, mu = F.norm_interp_f0(f0.copy(), "log", True)
-        assert np.array_equal(mu, ru.numpy()) and np.allclose(mf, rf.numpy(), rtol=0, atol=1e-6)
+        assert np.array_equal(mu, g[f"f0_{i}_uv"]) and np.allclose(mf, g[f"f0_{i}_norm"], rtol=0, atol=1e-6)
 
 
 def test_item_to_utterance_feeds_pack_batch():

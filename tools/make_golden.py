@@ -1,8 +1,8 @@
-"""Generate tests/golden/*.npz by executing the UNMODIFIED reference (build container only).
+"""Generate tests/golden/*.npz by executing the UNMODIFIED reference.
 
-    python tools/make_golden.py            # writes tests/golden/
+    STYLESINGER_REF=<checkout of AaronZ345/StyleSinger> python tools/make_golden.py [case ...]   # writes tests/golden/
 
-What it does (SURVEY.md §8c): imports /root/reference through tools/ref_import.py, builds the
+What it does (SURVEY.md §8c): imports the reference through tools/ref_import.py, builds the
 reference's own ``StyleSinger`` / ``HifiGanGenerator`` modules, loads the synthetic checkpoints of
 ``stylesinger_b200.synth`` with ``strict=True`` (which also proves state-dict name/shape
 compatibility with released checkpoints), monkey-patches ``torch.randn/randn_like/rand/rand_like``
@@ -246,10 +246,138 @@ def case_emotion_encoder(name, partials=5, seed=71):
     print("wrote", name, len(d), "arrays")
 
 
+def _put(d, alias, key, t):
+    """Store t under key, or record key as an alias of an identical array already stored (keeps the fixture small)."""
+    a = t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else np.asarray(t)
+    for k, v in d.items():
+        if isinstance(v, np.ndarray) and v.dtype == a.dtype and v.shape == a.shape and np.array_equal(v, a):
+            alias[key] = k
+            return
+    d[key] = a
+
+
+def case_dropin(name, T=8, seed=2024, utt=dict(seconds=0.3, utt_idx=11, ref_frames=32, phones=4)):
+    """The reference's own StyleSingerInfer.forward_model (predicted durations, use_nsf off, torch.randn* on
+    NoiseSource(seed)) on one synthetic item, recorded where stylesinger_b200.modules plugs in: the model call's inputs and
+    outputs, the first and last call of every module a registry-level drop-in replaces, and the vocoder's input and
+    waveform (tests/test_gpu_reference_dropin.py)."""
+    sys.path.insert(0, os.path.join(REPO, "baseline"))
+    import ref_harness
+    r = ref_harness.ReferenceRunner(T=T, device="cpu")
+    r.hp["use_nsf"] = False
+    u = synth.make_utterance(utt["seconds"], utt_idx=utt["utt_idx"], ref_frames=utt["ref_frames"], phones=utt["phones"])
+    item = r.item_from_utterance(u)
+    m = r.infer.model
+    calls = {}
+    hooks = []
+    for key, mod in (("model", m), ("encoder", m.encoder), ("decoder", m.decoder), ("diffnet", m.postdiff.denoise_fn),
+                     ("ddiffnet1", m.f0_gen._denoise_fn), ("ddiffnet2", m.f0_gen_inpainte._denoise_fn)):
+        hooks.append(mod.register_forward_hook(lambda mod_, a, k, o, key=key: calls.setdefault(key, []).append((a, k, o)),
+                                               with_kwargs=True))
+    get_style, spec2wav = m.get_style, r.infer.vocoder.spec2wav
+
+    def style_spy(encoder_out, ref_mels, ret, infer=False, global_steps=0):
+        out = get_style(encoder_out, ref_mels, ret, infer, global_steps)
+        calls.setdefault("get_style", []).append(((encoder_out.clone(), ref_mels.clone(), ret["ref_f0"].clone()), {}, out))
+        return out
+
+    def voc_spy(mel, **kw):
+        wav = spec2wav(mel, **kw)
+        calls["vocoder"] = [((torch.from_numpy(mel.copy()),), {}, torch.from_numpy(np.asarray(wav)))]
+        return wav
+
+    m.get_style, r.infer.vocoder.spec2wav = style_spy, voc_spy
+    with torch.no_grad(), patched_rng(NoiseSource(seed)):
+        wav = r.infer.forward_model(item)
+    for h in hooks:
+        h.remove()
+    r.close()
+    (ma, mk, ret), = calls.pop("model")
+    mk = dict(mk, txt_tokens=ma[0])
+    d, alias = {"wav": np.asarray(wav, np.float32)}, {}
+    for k in ("txt_tokens", "spk_embed", "emo_embed", "ref_mels", "ref_f0", "note", "note_dur", "note_type"):
+        _put(d, alias, "in_" + k, mk[k])
+    for k in ("mel2ph", "mel_out", "f0_denorm", "style", "decoder_inp", "pitch_pred"):
+        _put(d, alias, "ret_" + k, ret[k])
+    for key, cs in calls.items():
+        for i, (a, kw, o) in ((0, cs[0]), (1, cs[-1])) if len(cs) > 1 else ((0, cs[0]),):
+            for j, t in enumerate(a):
+                _put(d, alias, f"{key}{i}_a{j}", t)
+            for k, t in kw.items():
+                _put(d, alias, f"{key}{i}_k_{k}", t)
+            _put(d, alias, f"{key}{i}_out", o)
+    d["meta"] = json.dumps({"T": T, "seed": seed, "utt": utt, "global_steps": mk["global_steps"], "mel_vmin": r.hp["mel_vmin"],
+                            "mel_vmax": r.hp["mel_vmax"], "calls": {k: len(v) for k, v in calls.items()}, "alias": alias})
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **d)
+    print("wrote", name, {k: v.shape for k, v in d.items() if hasattr(v, "shape")}, json.loads(d["meta"]))
+
+
+def case_formats(name):
+    """The reference's own on-disk writers and pure host helpers on small seeded inputs (tests/test_formats_cpu.py):
+    utils/commons/indexed_datasets.py's builder output, utils/commons/ckpt_utils.py's load_ckpt choice among two
+    checkpoints, and utils/pitch_utils.py's norm_interp_f0."""
+    import importlib.util
+    import pickle
+    import tempfile
+    import types
+    import ref_import
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+
+    def ref_module(rel, stubs=()):
+        for s in stubs:
+            sys.modules.setdefault(s, types.ModuleType(s))
+        spec = importlib.util.spec_from_file_location("ref_" + os.path.basename(rel)[:-3], os.path.join(ref_import.REF, rel))
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+        return mod
+
+    from test_formats_cpu import _items
+    d = {}
+    tmp = tempfile.mkdtemp(prefix="ssb_golden_")
+    ids = ref_module("utils/commons/indexed_datasets.py")
+    b = ids.IndexedDatasetBuilder(os.path.join(tmp, "test"))
+    for it in _items():
+        b.add_item(it)
+    b.finalize()
+    for ext in ("data", "idx"):
+        d["ids_" + ext] = np.frombuffer(open(os.path.join(tmp, "test." + ext), "rb").read(), np.uint8)
+
+    ck = ref_module("utils/commons/ckpt_utils.py")
+
+    class Tiny(torch.nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.encoder = torch.nn.Linear(4, 3)
+            self.proj = torch.nn.Conv1d(3, 2, 3)
+
+    torch.manual_seed(0)
+    for step in (7, 3):
+        sd = Tiny().state_dict()
+        torch.save({"state_dict": {"model": sd}, "global_step": step}, os.path.join(tmp, f"model_ckpt_steps_{step}.ckpt"))
+        d.update({f"ckpt{step}_{k}": v.numpy() for k, v in sd.items()})
+    dst = Tiny()
+    ck.load_ckpt(dst, tmp, "model", strict=True)
+    d.update({f"loaded_{k}": v.numpy() for k, v in dst.state_dict().items()})
+
+    pu = ref_module("utils/pitch_utils.py", stubs=("librosa",))
+    rng = np.random.default_rng(1)
+    hp = {"pitch_norm": "log", "use_uv": True}
+    for i, (n, p0) in enumerate(((50, 0.3), (17, 0.0), (9, 1.0), (64, 0.9))):
+        f0 = rng.uniform(100, 600, n).astype(np.float32)
+        f0[rng.random(n) < p0] = 0.0
+        rf, ru = pu.norm_interp_f0(f0.copy(), hp)
+        d.update({f"f0_{i}": f0, f"f0_{i}_norm": rf.numpy(), f"f0_{i}_uv": ru.numpy()})
+    import shutil
+    shutil.rmtree(tmp)
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **d)
+    print("wrote", name, len(d), "arrays")
+
+
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # importing the reference must not write __pycache__ into its tree
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
-    which = sys.argv[1:] or ["small", "t25", "t100", "plms", "sched", "voc", "emo"]
+    which = sys.argv[1:] or ["small", "t25", "t100", "plms", "sched", "voc", "emo", "dropin", "formats"]
     if "small" in which:
         case_model("ref_small_T4", T=4, frames=96, phones=12, ref_frames=64, seed=11, utt_idx=100)
     if "t25" in which:
@@ -264,3 +392,7 @@ if __name__ == "__main__":
         case_vocoder("ref_vocoder_f24", frames=24, seed=31)
     if "emo" in which:
         case_emotion_encoder("ref_emotion_encoder")
+    if "dropin" in which:
+        case_dropin("ref_dropin_T8")
+    if "formats" in which:
+        case_formats("ref_formats")

@@ -1,8 +1,8 @@
 """Import shim for the UNMODIFIED reference (never for the product path).
 
-The reference lives at /root/reference in the build container and - staged byte for byte by tools/stage_reference.py -
-under baseline/_ref/StyleSinger on the GPU box.  Users: tools/make_golden.py (fixtures), baseline/ref_harness.py (the
-reference arms of bench.py and tools/baseline_arms.py) and tests/test_gpu_reference_dropin.py.  Shims follow SURVEY.md
+The reference is a checkout of AaronZ345/StyleSinger named by the STYLESINGER_REF environment variable; nothing in the
+package or the tests needs it.  Users: tools/make_golden.py (the fixtures under tests/golden/) and baseline/ref_harness.py
+(the reference arms of bench.py and tools/baseline_arms.py).  Shims follow SURVEY.md
 §8(c): they only satisfy import-time dependencies that are unused on the hot path (librosa, matplotlib, resemblyzer,
 parselmouth, skimage, webrtcvad, ... are imported by reference files but never called between `ph` tokens and the
 waveform); no hot-path arithmetic is touched.
@@ -17,10 +17,8 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def find_reference():
-    for c in (os.environ.get("STYLESINGER_REF"), "/root/reference", os.path.join(_REPO, "baseline", "_ref", "StyleSinger")):
-        if c and os.path.isdir(os.path.join(c, "modules", "StyleSinger")):
-            return c
-    return None
+    c = os.environ.get("STYLESINGER_REF")
+    return c if c and os.path.isdir(os.path.join(c, "modules", "StyleSinger")) else None
 
 
 REF = find_reference()
@@ -74,7 +72,7 @@ def install(T=100, f0_T=None, overrides=None):
     global _finder
     ref = find_reference()
     if ref is None:
-        raise RuntimeError("reference not found (STYLESINGER_REF, /root/reference or baseline/_ref/StyleSinger)")
+        raise RuntimeError("reference not found: set STYLESINGER_REF to a checkout of AaronZ345/StyleSinger")
     if ref not in sys.path:
         sys.path.insert(0, ref)
     os.chdir(ref)
